@@ -3,9 +3,13 @@
 (forward + both backwards + five Adam updates) on synthetic batches of the BASELINE configurations.
 
     python bench.py [--config C2|C3|C4|C5] [--gpus N] [--steps K] [--warmup W] [--skip-prob P] [--strong] [--impl reference]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  --dump-outputs DIR (rank 0) writes what the last of the K timed steps handed its caller
+as DIR/<name>.npy, float32: the four losses, every module's updated parameters and their gradients, and the BatchNorm
+running statistics (see dump_outputs).  The inputs (weights, batch, noise, skip draws) are seeded, so two builds run
+with the same arguments can be compared output for output.
   value       device-timed throughput (CUDA events, max over ranks) of K graph-replayed steps, batch resident in HBM
   e2e         the same through the public drop-in API (p2pvg_b200.data.DevicePrefetcher feeding
               models.p2p_model.P2PModel.__call__): every step's batch is copied from pinned host memory inside the timed
@@ -131,6 +135,43 @@ class ClockSampler:
 
 def log(msg):
     print(f"[bench {time.strftime('%H:%M:%S')}] {msg}", file=sys.stderr, flush=True)
+
+
+DUMP_LIMIT = 64_000_000   # bytes --dump-outputs may write in all
+DUMP_WHOLE = 4096         # arrays up to this many elements are always written whole
+
+
+def step_outputs(eng, losses):
+    """What one train step hands its caller (P2PModel exposes the parameters and their .grad as views of the engine's
+    arenas): the losses, per module every updated parameter and its gradient, and the BatchNorm running statistics."""
+    arrays = {"losses": losses}
+    for m, A in eng.arena.items():
+        for k in A.names:
+            arrays[f"{m}.{k}"] = A.p[k]
+            arrays[f"{m}.{k}.grad"] = A.g[k]
+        arrays.update({f"{m}.{k}": v for k, v in eng.buffers[m].items() if v.is_floating_point()})
+    return {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy (float32), DUMP_LIMIT bytes at most.  If the arrays are larger than that
+    together, each one of more than DUMP_WHOLE elements is replaced by the same fraction of its flattened elements, in
+    index order, at indices drawn from a fixed seed: every run and every build samples the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    header = 128   # bytes of a .npy header for these shapes
+    room = (DUMP_LIMIT - len(arrays) * (header + 4 * (DUMP_WHOLE + 1))) // 4
+    frac = min(1.0, room / sum(a.size for a in arrays.values()))
+    written = 0
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        keep = min(a.size, max(DUMP_WHOLE, int(a.size * frac)))
+        if keep < a.size:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        path = os.path.join(out_dir, f"{name}.npy")
+        np.save(path, a)
+        written += os.path.getsize(path)
+    assert written <= DUMP_LIMIT, written
+    log(f"wrote {len(arrays)} arrays ({written / 1e6:.1f} MB, {100 * frac:.0f}% of the elements of the large ones) to {out_dir}")
 
 
 def oracle_cfg(c):
@@ -278,7 +319,10 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-library", action="store_true")
     ap.add_argument("--skip-phases", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     c = CONFIGS[args.config]
     if args.impl == "reference":
         return run_reference(args, c)
@@ -353,11 +397,13 @@ def main():
     e0.record()
     executed = 0
     for _ in range(args.steps):
-        eng.step(x_dev, use_graph=use_graph, return_device=True)
+        out = eng.step(x_dev, use_graph=use_graph, return_device=True)
         executed += eng.last_plan.S
     e1.record()
     barrier()
     tw1 = time.time()
+    if args.dump_outputs and rank == 0:   # now: every later step trains the same model on and reuses the loss buffer
+        dump_outputs(args.dump_outputs, step_outputs(eng, out))
     launches = K.launches - n0
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:

@@ -10,18 +10,30 @@
                        hundred KB; the checkpoint format does not depend on the backbone)
   ckpt_ref_small_next.pt   the batch / eps / skip draws and the four losses of the reference's NEXT step from that
                        checkpoint (resume check), plus digests of the checkpointed tensors.
+  ckpt_ref_resume.pt   the reverse direction: a checkpoint written by the drop-in ``P2PModel.save`` (ckpt_ref_small.pth
+                       loaded, saved as epoch 9) loaded by the reference's own ``P2PModel.load`` under stock
+                       ``torch.optim.Adam``, then one Adam step with all gradients set to one.  Stores the reference's
+                       module layout (state_dict keys / shapes, parameter order), the epoch ``load`` returned, and the
+                       Adam step counts and digests of the parameters after that step.
+  init_sha256.json     for every case of make_golden.py, the SHA-256 of each floating-point tensor of the reference's
+                       freshly initialised modules (float32 bytes): pins the initial weights bit for bit, whatever order
+                       a sum over them would be taken in.
 
-    python tests/golden/make_golden_extra.py
+    python tests/golden/make_golden_extra.py [gen] [ckpt] [resume] [init]     (default: all)
 """
+import hashlib
+import json
 import os
+import subprocess
 import sys
+import tempfile
 
 import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
-from make_golden import LegacyAdam, ROOT, import_reference, make_opt  # noqa: E402
+from make_golden import CASES, LegacyAdam, ROOT, import_reference, make_opt  # noqa: E402
 
 sys.path.insert(0, ROOT)
 from oracle.p2p_oracle import tensor_digest  # noqa: E402
@@ -135,12 +147,75 @@ def run_ckpt_case(p2p_model, backbones):
     print("wrote", path, os.path.getsize(path) // 1024, "KiB; next-step losses", losses)
 
 
+def run_resume_case(p2p_model, backbones):
+    with tempfile.TemporaryDirectory() as tmp:
+        dropin_pth = os.path.join(tmp, "dropin.pth")
+        # the drop-in and the reference both own the package names `models` / `misc`: write the drop-in checkpoint in a
+        # process of its own
+        subprocess.check_call([sys.executable, "-c", "import sys; sys.path.insert(0, sys.argv[1]); "
+                               "from tests.test_generate_ckpt_golden import small_model, GOLD; import os; m, _ = small_model(); "
+                               "m.load(os.path.join(GOLD, 'ckpt_ref_small.pth')); m.save(sys.argv[2], 9)", ROOT, dropin_pth])
+        states = torch.load(dropin_pth, weights_only=False)
+    side = torch.load(os.path.join(HERE, "ckpt_ref_small_next.pt"), weights_only=False)
+    cfg, B = side["cfg"], side["B"]
+    torch.manual_seed(11)
+    opt = make_opt(backbones["mlp"], dataset="h36m", batch_size=B)
+    model = p2p_model.P2PModel(B, 1, cfg["g_dim"], cfg["z_dim"], cfg["rnn_size"], 1, 1, 2, opt=opt)   # stock torch.optim.Adam
+    mods = ("frame_predictor", "posterior", "prior", "encoder", "decoder")
+    layout = {m: dict(state=[(k, tuple(v.shape)) for k, v in getattr(model, m).state_dict().items()],
+                      params=[k for k, _ in getattr(model, m).named_parameters()]) for m in mods}
+    # torch >= 2.6 defaults torch.load to weights_only=True, which the reference's load(pth) does not survive for a
+    # checkpoint carrying the pickled opt namespace: hand it the states instead
+    epoch = model.load(states=states)
+    adam = {}
+    for m in mods:
+        o = getattr(model, m + "_optimizer")
+        assert type(o) is torch.optim.Adam
+        adam[m] = dict(lr=o.param_groups[0]["lr"], betas=tuple(o.param_groups[0]["betas"]))
+        for p in getattr(model, m).parameters():
+            p.grad = torch.ones_like(p)
+        o.step()
+    fix = dict(cfg=cfg, B=B, saved_epoch=9, start_epoch=epoch, layout=layout, adam=adam,
+               steps={m: [int(v["step"]) for v in getattr(model, m + "_optimizer").state_dict()["state"].values()] for m in mods},
+               post={m: {k: tensor_digest(v) for k, v in getattr(model, m).named_parameters()} for m in mods})
+    path = os.path.join(HERE, "ckpt_ref_resume.pt")
+    torch.save(fix, path)
+    print("wrote", path, os.path.getsize(path) // 1024, "KiB; start epoch", epoch)
+
+
+def sha256_f32(t):
+    return hashlib.sha256(t.detach().to(torch.float32).contiguous().numpy().tobytes()).hexdigest()
+
+
+def run_init_case(p2p_model, backbones):
+    out = {}
+    for name, spec in CASES.items():
+        torch.manual_seed(1)   # the construction of make_golden.run_case
+        opt = make_opt(backbones[spec["width"]], **spec["opt"])
+        if opt.batch_size is None:
+            opt.batch_size = spec["B"]
+        model = p2p_model.P2PModel(opt.batch_size, spec["channels"], 128, 10, 256, 1, 1, 2, opt=opt)
+        out[name] = {m: {k: sha256_f32(v) for k, v in getattr(model, m).state_dict().items() if v.is_floating_point()}
+                     for m in ("frame_predictor", "posterior", "prior", "encoder", "decoder")}
+    path = os.path.join(HERE, "init_sha256.json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=0, sort_keys=True)
+    print("wrote", path, os.path.getsize(path) // 1024, "KiB")
+
+
 def main():
+    parts = sys.argv[1:] or ["gen", "ckpt", "resume", "init"]
     torch.set_num_threads(8)
     p2p_model, backbones = import_reference()
-    for name, spec in GEN_CASES.items():
-        run_gen_case(name, spec, p2p_model, backbones)
-    run_ckpt_case(p2p_model, backbones)
+    if "gen" in parts:
+        for name, spec in GEN_CASES.items():
+            run_gen_case(name, spec, p2p_model, backbones)
+    if "ckpt" in parts:
+        run_ckpt_case(p2p_model, backbones)
+    if "resume" in parts:
+        run_resume_case(p2p_model, backbones)
+    if "init" in parts:
+        run_init_case(p2p_model, backbones)
 
 
 if __name__ == "__main__":

@@ -2,10 +2,10 @@
 tests/golden/make_golden_extra.py from the unmodified reference: eval-mode BatchNorm, model_mode in {full, posterior,
 prior}, skip_frame in {False, True}).  (2) Checkpoint round trip with the reference's own save / load
 (models/p2p_model.py:289-330): a reference-written .pth loads into the drop-in P2PModel; a drop-in-written .pth loads
-into the reference's modules and resumes under stock torch.optim.Adam.  CPU only."""
+into the reference's modules and resumes under stock torch.optim.Adam (tests/golden/ckpt_ref_resume.pt, written by
+tests/golden/make_golden_extra.py).  CPU only."""
 import glob
 import os
-import sys
 import types
 
 import numpy as np
@@ -77,44 +77,43 @@ def test_reference_checkpoint_loads_into_dropin():
     assert getattr(model.opt, "backbone_net", 0) != 0, "load() must keep the live backbone module (the pickled opt holds 0)"
 
 
-REF = os.environ.get("P2PVG_REF", "/root/reference")
+def reference_load(states, layout, adam):
+    """What the reference's ``P2PModel.load(states=...)`` (models/p2p_model.py:310-330) does with a checkpoint, on the
+    reference's module layout recorded in tests/golden/ckpt_ref_resume.pt: a strict ``load_state_dict`` of each of the five
+    modules, then ``torch.optim.Adam.load_state_dict`` of its optimiser, built over the module's parameters in registration
+    order.  Returns (start epoch, {module: {parameter name: Parameter}}, {module: Adam})."""
+    params, optims = {}, {}
+    for m in MODULES:
+        sd = states[m]
+        want = dict(layout[m]["state"])
+        assert set(sd) == set(want), f"{m}: missing {sorted(set(want) - set(sd))}, unexpected {sorted(set(sd) - set(want))}"
+        for k, shape in want.items():
+            assert tuple(sd[k].shape) == shape, f"{m}.{k}: {tuple(sd[k].shape)} != {shape}"
+        params[m] = {k: torch.nn.Parameter(sd[k].detach().clone().float()) for k in layout[m]["params"]}
+        optims[m] = torch.optim.Adam(params[m].values(), lr=adam[m]["lr"], betas=adam[m]["betas"])
+        optims[m].load_state_dict(states[m + "_opt"])
+    return states["epoch"] + 1, params, optims
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout only exists in the build container")
 def test_dropin_checkpoint_loads_into_reference_and_resumes_under_stock_adam(tmp_path):
-    """drop-in save() -> reference load(): run in a subprocess so that the reference's `models` / `misc` packages do not
-    shadow anything in this process."""
-    import subprocess
+    """drop-in save() -> the reference's load() under stock torch.optim.Adam, and one resumed Adam step that matches the
+    one the reference took from the same checkpoint (tests/golden/ckpt_ref_resume.pt)."""
+    fix = torch.load(os.path.join(GOLD, "ckpt_ref_resume.pt"), weights_only=False)
     model, side = small_model()
     model.load(os.path.join(GOLD, "ckpt_ref_small.pth"))
     out = str(tmp_path / "dropin.pth")
-    model.save(out, 9)
-    code = f'''
-import sys, types, torch
-sys.path.insert(0, {os.path.join(os.path.dirname(__file__), "golden")!r})
-from make_golden import import_reference, make_opt
-p2p_model, backbones = import_reference()
-torch.manual_seed(11)
-opt = make_opt(backbones["mlp"], dataset="h36m", batch_size={side["B"]})
-cfg = {side["cfg"]!r}
-m = p2p_model.P2PModel({side["B"]}, 1, cfg["g_dim"], cfg["z_dim"], cfg["rnn_size"], 1, 1, 2, opt=opt)   # stock torch.optim.Adam
-# torch >= 2.6 defaults torch.load to weights_only=True, which the reference's load(pth) (written for torch 1.0) does not
-# survive for ANY checkpoint carrying the pickled opt namespace: use its own `states=` entry instead
-epoch = m.load(states=torch.load({out!r}, weights_only=False))
-assert epoch == 10, epoch
-ref = torch.load({os.path.join(GOLD, "ckpt_ref_small.pth")!r}, weights_only=False)
-for mod in ("frame_predictor", "posterior", "prior", "encoder", "decoder"):
-    sd = getattr(m, mod).state_dict()
-    for k, v in ref[mod].items():
-        assert torch.equal(sd[k], v), (mod, k)
-    o = getattr(m, mod + "_optimizer")
-    assert isinstance(o, torch.optim.Adam)
-    for p in getattr(m, mod).parameters():
-        p.grad = torch.ones_like(p)
-    o.step()     # ADVICE r01: must not raise KeyError('weight_decay' / 'amsgrad' ...)
-    st = o.state_dict()["state"]
-    assert all(int(v["step"]) == 2 for v in st.values()), [int(v["step"]) for v in st.values()][:3]
-print("OK")
-'''
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "OK" in r.stdout, r.stdout + r.stderr
+    model.save(out, fix["saved_epoch"])
+    states = torch.load(out, weights_only=False)
+    epoch, params, optims = reference_load(states, fix["layout"], fix["adam"])
+    assert epoch == fix["start_epoch"] == 10, epoch
+    ref = torch.load(os.path.join(GOLD, "ckpt_ref_small.pth"), weights_only=False)
+    for m in MODULES:
+        for k, v in ref[m].items():
+            assert torch.equal(states[m][k], v), (m, k)
+        for p in params[m].values():
+            p.grad = torch.ones_like(p)
+        optims[m].step()     # must not raise KeyError('weight_decay' / 'amsgrad' ...)
+        steps = [int(v["step"]) for v in optims[m].state_dict()["state"].values()]
+        assert steps == fix["steps"][m] and all(s == 2 for s in steps), steps[:3]
+        for k, d in fix["post"][m].items():
+            check_digest(params[m][k], d, 1e-6, 1e-9, f"{m}.{k} after the resumed Adam step")
