@@ -126,17 +126,6 @@ int p2pvg_upsample2_fwd(const void* x, void* y, int dtype, int N, int H, int W, 
 int p2pvg_upsample2_bwd(const void* dy, void* dx, int dtype, int N, int H, int W, int C, void* stream);
 int p2pvg_gather_add(void* dst, int dtype, const float* src, const int* grp_src, int G, int64_t n, void* stream);
 
-/* Thin ends of the dcgan stacks (1 or 3 image channels on one side; HBM-bound direct kernels, fp32 master weights):
- *   conv_thin_in : y[N,H/2,W/2,Co] = conv4x4/s2/p1(x[N,H,W,Ci<=4]) . w[Co][Ci][4][4] + bias   — encoder c1 forward
- *                  (models/dcgan_64.py:34) and the data-gradient of the last decoder layer (its ConvT weight [Cin][nc][4][4]
- *                  has this layout with Co = Cin)
- *   convT_thin_out: y[N,2H,2W,Co<=3] = convT4x4/s2/p1(x[N,H,W,Ci]) . w[Ci][Co][4][4] + bias + addend[src] — last decoder layer
- *                  forward (models/dcgan_64.py:76); y_dtype = the activation dtype or fp32 (for the skip addend). */
-int p2pvg_conv_thin_in(const void* x, int dtype, const float* w, const float* bias, void* y, int N, int H, int W, int Ci, int Co,
-                       void* stream);
-int p2pvg_convT_thin_out(const void* x, int dtype, const float* w, const float* bias, const float* addend, const int* grp_src,
-                         int imgs_per_group, void* y, int y_dtype, int N, int H, int W, int Ci, int Co, void* stream);
-
 /* 4x4 / stride 2 / pad 1 lowering (nn.Conv2d(nin,nout,4,2,1), models/dcgan_64.py:8; and the data-gradient of
  * nn.ConvTranspose2d(nin,nout,4,2,1), models/dcgan_64.py:20): x [N,H,W,C] -> col [N*H/2*W/2, 16*C], K order (kh,kw,c). */
 int p2pvg_im2col_k4s2p1(const void* x, void* col, int dtype, int N, int H, int W, int C, void* stream);
@@ -203,8 +192,8 @@ int p2pvg_lstm_pointwise_bwd(const float* dh, const float* dc_next, const float*
  * timesteps).  tf32 = 1 dispatches by hidden size: R in {64,128,256}: thread-block clusters of 8 CTAs, hardware cluster barrier per
  * timestep; R = 512: clusters of 16 CTAs (non-portable size), slabs of 16 / 32 / 48 batch rows per cluster chosen so that the
  * resident clusters cover the batch in one wave, backward reduction scattered through distributed shared memory, the part of the
- * weight slice that does not fit the registers in shared memory (16-row slabs) or tensor memory (larger slabs).  tf32 = 0 (and
- * P2PVG_LSTM_CLUSTER=0): cooperative grid with a grid barrier per timestep, exact fp32 FFMA products.
+ * weight slice that does not fit the registers in shared memory (16-row slabs) or tensor memory (larger slabs).  tf32 = 0, or
+ * tf32 = 1 with R not in {64,128,256,512}: cooperative grid with a grid barrier per timestep, exact fp32 FFMA products.
  *   forward : gates_s = pre_s + b_hh + h_{s-1}.W_hh^T -> (i,f,g,o) -> c_s, h_s       pre [S,B,4R] = x-part incl. b_ih
  *             gates [S,B,4R] out (activations), hs / cs [S+1,B,R] with slot 0 = initial state (zeros, models/lstm.py:21-27)
  *   backward: dh_s = dhtop_s + dG_{s+1}.W_hh, cell backward -> dG [S,B,4R] (gradient w.r.t. the gate pre-activations)

@@ -185,13 +185,6 @@ class CudaKernels:
                                           _i(Cn), _i(Cm), _p(bias), _p(addend), _p(grp_src), _i(imgs_per_group), _i(int(accumulate)),
                                           _p(ws), _sz(ws.numel()), fusion, self._stream()))
 
-    def conv_thin_in(self, x, w, bias, y, N, H, W, Ci, Co):
-        self._ck(self.lib.p2pvg_conv_thin_in(_p(x), _i(_dt(x)), _p(w), _p(bias), _p(y), _i(N), _i(H), _i(W), _i(Ci), _i(Co), self._stream()))
-
-    def convT_thin_out(self, x, w, bias, y, N, H, W, Ci, Co, addend=None, grp_src=None, imgs_per_group=0):
-        self._ck(self.lib.p2pvg_convT_thin_out(_p(x), _i(_dt(x)), _p(w), _p(bias), _p(addend), _p(grp_src), _i(imgs_per_group), _p(y),
-                                               _i(_dt(y)), _i(N), _i(H), _i(W), _i(Ci), _i(Co), self._stream()))
-
     # -- conv lowering ---------------------------------------------------------------------
     def im2col(self, x, col, N, H, W, C):
         self._ck(self.lib.p2pvg_im2col_k4s2p1(_p(x), _p(col), _i(_dt(x)), _i(N), _i(H), _i(W), _i(C), self._stream()))

@@ -4,7 +4,6 @@
 #include <string.h>
 
 #include "../../include/p2pvg_b200.h"
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -39,9 +38,6 @@ int p2pvg_layernorm_fwd_impl(const float*, const float*, const float*, float*, f
 int p2pvg_layernorm_bwd_impl(const float*, const float*, const float*, const float*, const float*, float*, float*, float*, long long, int,
                              void*, size_t, cudaStream_t);
 int p2pvg_mse_plain_impl(const float*, const float*, const int*, const float*, int, long long, float*, float*, int, cudaStream_t);
-int p2pvg_conv_thin_in_impl(const void*, int, const float*, const float*, void*, int, int, int, int, int, cudaStream_t);
-int p2pvg_convT_thin_out_impl(const void*, int, const float*, const float*, const float*, const int*, int, void*, int, int, int, int, int,
-                              int, cudaStream_t);
 int p2pvg_conv_gemm_impl(int, const void*, const void*, long long, void*, int, long long, int, int, int, int, int, int, const float*,
                          const float*, const int*, int, int, void*, size_t, void*, int, cudaStream_t);
 int p2pvg_bn_fwd_finalize_tiles_impl(const void*, int, int, int, int, long long, int, const float*, const float*, float, float*, float*, float*,
@@ -160,15 +156,6 @@ int p2pvg_conv_gemm(int kind, const void* a, const void* b, int64_t ldb, void* c
                               imgs_per_group, accumulate, workspace, ws_bytes, fwd_stat, add_dt, ST);
 }
 
-int p2pvg_conv_thin_in(const void* x, int dtype, const float* w, const float* bias, void* y, int N, int H, int W, int Ci, int Co,
-                       void* stream) {
-  return p2pvg_conv_thin_in_impl(x, dtype, w, bias, y, N, H, W, Ci, Co, ST);
-}
-int p2pvg_convT_thin_out(const void* x, int dtype, const float* w, const float* bias, const float* addend, const int* grp_src,
-                         int imgs_per_group, void* y, int y_dtype, int N, int H, int W, int Ci, int Co, void* stream) {
-  return p2pvg_convT_thin_out_impl(x, dtype, w, bias, addend, grp_src, imgs_per_group, y, y_dtype, N, H, W, Ci, Co, ST);
-}
-
 int p2pvg_im2col_k4s2p1(const void* x, void* col, int dtype, int N, int H, int W, int C, void* stream) {
   return p2pvg_im2col_k4s2p1_impl(x, col, dtype, N, H, W, C, ST);
 }
@@ -264,24 +251,18 @@ int p2pvg_lstm_pointwise_bwd(const float* dh, const float* dc_next, const float*
                              float* dgates, float* dc_prev, int B, int R, void* stream) {
   return p2pvg_lstm_pointwise_bwd_impl(dh, dc_next, gates, c_prev, c, dgates, dc_prev, B, R, ST);
 }
-// tensor-core mode: thread-block-cluster scans (lstm_cluster.cu) for R in {64,128,256}, lstm_cluster512.cu for R = 512; P2PVG_LSTM_CLUSTER=0 keeps the
-// cooperative-grid scans, which also serve the exact-fp32 mode
-static bool cluster_scan_enabled() {
-  static const int off = [] { const char* e = getenv("P2PVG_LSTM_CLUSTER"); return (e != nullptr && e[0] == '0') ? 1 : 0; }();
-  return !off;
-}
-// R = 512 (BASELINE config 5) runs on clusters of 16 CTAs (lstm_cluster512.cu)
-static bool use_cluster_scan(int R) { return cluster_scan_enabled() && p2pvg_lstm_cluster_supported(R); }
+// tensor-core mode: thread-block-cluster scans, lstm_cluster.cu for R in {64,128,256} and lstm_cluster512.cu (clusters of 16
+// CTAs) for R = 512 (BASELINE config 5); the cooperative-grid scans serve the exact-fp32 mode and every other R
 int p2pvg_lstm_scan_fwd(const float* pre, const float* whh, const float* bhh, float* gates, float* hs, float* cs, int S, int B, int R,
                         int tf32, unsigned* counter, void* stream) {
-  if (tf32 && R == 512 && cluster_scan_enabled()) return p2pvg_lstm_cluster512_fwd_impl(pre, whh, bhh, gates, hs, cs, S, B, ST);
-  if (tf32 && use_cluster_scan(R)) return p2pvg_lstm_cluster_fwd_impl(pre, whh, bhh, gates, hs, cs, S, B, R, ST);
+  if (tf32 && R == 512) return p2pvg_lstm_cluster512_fwd_impl(pre, whh, bhh, gates, hs, cs, S, B, ST);
+  if (tf32 && p2pvg_lstm_cluster_supported(R)) return p2pvg_lstm_cluster_fwd_impl(pre, whh, bhh, gates, hs, cs, S, B, R, ST);
   return p2pvg_lstm_scan_fwd_impl(pre, whh, bhh, gates, hs, cs, S, B, R, tf32, counter, ST);
 }
 int p2pvg_lstm_scan_bwd(const float* dhtop, const float* whh, const float* gates, const float* cs, float* dG, int S, int B, int R,
                         int tf32, unsigned* counter, void* stream) {
-  if (tf32 && R == 512 && cluster_scan_enabled()) return p2pvg_lstm_cluster512_bwd_impl(dhtop, whh, gates, cs, dG, S, B, ST);
-  if (tf32 && use_cluster_scan(R)) return p2pvg_lstm_cluster_bwd_impl(dhtop, whh, gates, cs, dG, S, B, R, ST);
+  if (tf32 && R == 512) return p2pvg_lstm_cluster512_bwd_impl(dhtop, whh, gates, cs, dG, S, B, ST);
+  if (tf32 && p2pvg_lstm_cluster_supported(R)) return p2pvg_lstm_cluster_bwd_impl(dhtop, whh, gates, cs, dG, S, B, R, ST);
   return p2pvg_lstm_scan_bwd_impl(dhtop, whh, gates, cs, dG, S, B, R, tf32, counter, ST);
 }
 int p2pvg_lstm_cluster512_max_clusters(int which) { return p2pvg_lstm_cluster512_max_clusters_impl(which); }

@@ -15,7 +15,6 @@
 // kind 3  y[N,H,W,Cn] = conv3x3_s1_p1(x[N,H,W,Ck]) . W[Cn, (tap, Ck)] + bias + addend      vgg layer forward (kind 0 geometry, 9 taps)
 // kind 4  g[Cm, (tap, Cn)] = sum_pix a[pix, Cm]^T . gather_3x3(b)[pix, tap, Cn]             vgg weight gradients (kind 1 geometry)
 // kind 5  kind 3 with mirrored tap offsets (pixel - (kh-1, kw-1)): the data gradient of a 3x3 convolution
-#include <cstdlib>
 #include <mutex>
 
 #include "tc_common.cuh"
@@ -761,15 +760,12 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 EncodeTiledFn g_enc = nullptr;
 std::once_flag g_once2;
 int g_sms = 148;
-int g_k1_wide_max = 1 << 30;  // kind 1: 256-wide tiles while there are at most this many 128-wide output tiles (P2PVG_K1_WIDE_MAX)
-int g_bn256 = 1;  // P2PVG_CONV_BN256=0 keeps the 128-wide tiles (A/B comparison)
 int g_attr[2][3][3] = {};
-int g_convt4_max_cn = 64;   // kind 2 with at most this many output channels: the four parity phases fused into one tile (P2PVG_CONVT4_MAX_CN;
-                            // 0 = off).  Measured (C2 step, B200): 64 -> -0.36 ms; 128 -> +0.1 ms (the N = 64 MMAs of the fused tile issue twice as
-                            // many instructions as the 128-wide phase tiles, which outweighs the saved operand fills)
+// kind 2 with at most this many output channels: the four parity phases fused into one tile.  Measured (C2 step, B200):
+// 64 -> -0.36 ms; 128 -> +0.1 ms (the N = 64 MMAs of the fused tile issue twice as many instructions as the 128-wide phase
+// tiles, which outweighs the saved operand fills)
+constexpr int kConvt4MaxCn = 64;
 int g_convt4_attr[2] = {};
-int g_bres = 1;      // 64 -> 64 channel 3x3 layers: weights resident in shared memory (P2PVG_CONV_BRES=0 disables)
-int g_k1_swap = 1;   // kind 1 / 4 with 64 output channels: swapped operand roles (P2PVG_K1_SWAP=0 disables)
 
 void resolve2() {
   int dev = 0, sms = 0;
@@ -779,16 +775,6 @@ void resolve2() {
   if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
     g_enc = reinterpret_cast<EncodeTiledFn>(fn);
   (void)cudaGetLastError();
-  const char* e = getenv("P2PVG_CONV_BN256");
-  if (e != nullptr && e[0] == '0') g_bn256 = 0;
-  const char* br = getenv("P2PVG_CONV_BRES");
-  if (br != nullptr && br[0] == '0') g_bres = 0;
-  const char* sw = getenv("P2PVG_K1_SWAP");
-  if (sw != nullptr && sw[0] == '0') g_k1_swap = 0;
-  const char* f4 = getenv("P2PVG_CONVT4_MAX_CN");
-  if (f4 != nullptr) g_convt4_max_cn = atoi(f4);
-  const char* w = getenv("P2PVG_K1_WIDE_MAX");
-  if (w != nullptr) g_k1_wide_max = atoi(w);
 }
 
 int map2d(CUtensorMap* m, const void* base, long long dim0, long long dim1, long long ld, int box1) {
@@ -936,11 +922,11 @@ int p2pvg_conv_gemm_impl(int kind, const void* a, const void* b, long long ldb, 
     g.M = (int)pix; g.Ntot = Cn;
     rc = map4d(&ta, a, N, g.st * H, g.st * W, Ck, W, g.bh128, g.bn128, g.st);
     if (rc) return rc;
-    const int BN = (Cn % 256 == 0 && g_bn256) ? 256 : Cn > 64 ? 128 : 64;
+    const int BN = Cn % 256 == 0 ? 256 : Cn > 64 ? 128 : 64;
     rc = map2d(&tb, b, (long long)taps * Ck, Cn, ldb, BN);
     if (rc) return rc;
     const int nkb = taps * (Ck / 64);
-    g.bres = (BN == 64 && Cn == 64 && Ck == 64 && taps <= 9 && g_bres) ? 1 : 0;
+    g.bres = (BN == 64 && Cn == 64 && Ck == 64 && taps <= 9) ? 1 : 0;
     if (BN == 256) return launch<0, 256>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
     if (BN == 128) return launch<0, 128>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
     return launch<0, 64>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
@@ -952,10 +938,10 @@ int p2pvg_conv_gemm_impl(int kind, const void* a, const void* b, long long ldb, 
     rc = map2d(&tb, b, 16LL * Cn, Ck, ldb, 64);  // MN-major weight [Ck rows][16*Cn]
     if (rc) return rc;
     const int nkb = 4 * (Ck / 64);
-    if (Cn % 64 == 0 && Cn <= g_convt4_max_cn && !accumulate && (ldc % 16 == 0) && (c_dtype == P2PVG_F32 || ldc % 32 == 0) &&
+    if (Cn % 64 == 0 && Cn <= kConvt4MaxCn && !accumulate && (ldc % 16 == 0) && (c_dtype == P2PVG_F32 || ldc % 32 == 0) &&
         ((uintptr_t)c & 31) == 0 && (addend == nullptr || ((uintptr_t)addend & 15) == 0))
       return launch_convt4(ta, tb, c, c_dtype, ldc, g, bias, addend, grp_src, stat_partial, st);
-    const int BN = (Cn % 256 == 0 && g_bn256) ? 256 : Cn > 64 ? 128 : 64;
+    const int BN = Cn % 256 == 0 ? 256 : Cn > 64 ? 128 : 64;
     if (BN == 256) return launch<2, 256>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
     if (BN == 128) return launch<2, 128>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
     return launch<2, 64>(ta, tb, c, c_dtype, ldc, g, accumulate, bias, addend, grp_src, nullptr, 1, nkb, st, stat_partial);
@@ -967,7 +953,7 @@ int p2pvg_conv_gemm_impl(int kind, const void* a, const void* b, long long ldb, 
   // 64 output channels would fill only half of a 128-row MMA tile: swap the operand roles (M = taps*Cn from the gathered map,
   // N = Cm); the partial sums are then [taps*Cn][Cm] and the split-K reduce kernel writes the transposed result
   const int nkb = (int)((pix + 63) / 64);
-  g.swap = (Cm == 64 && g_k1_swap && nkb >= 16 && ws != nullptr && (size_t)2 * taps * Cn * Cm * sizeof(float) <= ws_bytes) ? 1 : 0;
+  g.swap = (Cm == 64 && nkb >= 16 && ws != nullptr && (size_t)2 * taps * Cn * Cm * sizeof(float) <= ws_bytes) ? 1 : 0;
   if (g.swap) {
     g.M = taps * Cn; g.Ntot = Cm;
     rc = map4d(&ta, b, N, g.st * H, g.st * W, Cn, g.bw64, g.bh64, g.bn64, g.st);
@@ -981,9 +967,8 @@ int p2pvg_conv_gemm_impl(int kind, const void* a, const void* b, long long ldb, 
     rc = map4d(&tb, b, N, g.st * H, g.st * W, Cn, g.bw64, g.bh64, g.bn64, g.st);
     if (rc) return rc;
   }
-  // a wide tile spans several filter taps when Cn == 64; 256-wide tiles pay off while there are few output tiles (measured)
-  const bool wide = !g.swap && g.Ntot % 256 == 0 && g_bn256 && (long long)cdiv(Cm, BLOCK_M) * (g.Ntot / 128) <= g_k1_wide_max;
-  const int BN = wide ? 256 : (g.Ntot % 128 == 0) ? 128 : 64;
+  // a wide tile spans several filter taps when Cn == 64
+  const int BN = (!g.swap && g.Ntot % 256 == 0) ? 256 : (g.Ntot % 128 == 0) ? 128 : 64;
   const long long tiles = (long long)cdiv(g.M, BLOCK_M) * cdiv(g.Ntot, BN);
   // split-K chosen by a small cost model (units: time of one 128x128x64 k-block on one SM, ~0.22 us): the persistent grid
   // processes ceil(items / SMs) rounds of (k-blocks per item + fixed per-item cost); partial sums cost a write + read

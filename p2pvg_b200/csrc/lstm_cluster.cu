@@ -17,8 +17,6 @@
 //
 //   forward :  gates_s = Pre_s + b_hh + h_{s-1} . W_hh^T ; (i,f,g,o) -> c_s, h_s
 //   backward:  dh_s = dHtop_s + dG_{s+1} . W_hh ; cell pointwise backward -> dG_s, dc_{s-1}
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace {
@@ -393,17 +391,14 @@ int p2pvg_lstm_cluster_max_clusters_impl(int which) {
   return n;
 }
 
-// rows per slab: 32 (MT = 2) above this batch size.  P2PVG_LSTM_MT2_ABOVE overrides (experiments).
-static int mt2_above() {
-  static const int v = [] { const char* e = getenv("P2PVG_LSTM_MT2_ABOVE"); return e ? atoi(e) : 128; }();
-  return v;
-}
+// rows per slab: 32 (MT = 2) above this batch size
+constexpr int kMt2Above = 128;
 
 // 8 clusters of 8 CTAs are co-resident on a B200 (measured): slabs of 32 rows keep up to 256 rows in one wave
 int p2pvg_lstm_cluster_fwd_impl(const float* pre, const float* whh, const float* bhh, float* gates, float* hs, float* cs, int S, int B,
                                 int R, cudaStream_t st) {
   if (S <= 0 || B <= 0) return P2PVG_OK;
-  const bool two = B > mt2_above();
+  const bool two = B > kMt2Above;
   switch (R) {
     case 64: return two ? launch_fwd<64, 2>(pre, whh, bhh, gates, hs, cs, S, B, st) : launch_fwd<64, 1>(pre, whh, bhh, gates, hs, cs, S, B, st);
     case 128: return two ? launch_fwd<128, 2>(pre, whh, bhh, gates, hs, cs, S, B, st) : launch_fwd<128, 1>(pre, whh, bhh, gates, hs, cs, S, B, st);
@@ -416,7 +411,7 @@ int p2pvg_lstm_cluster_fwd_impl(const float* pre, const float* whh, const float*
 int p2pvg_lstm_cluster_bwd_impl(const float* dhtop, const float* whh, const float* gates, const float* cs, float* dG, int S, int B, int R,
                                 cudaStream_t st) {
   if (S <= 0 || B <= 0) return P2PVG_OK;
-  const bool two = B > mt2_above();
+  const bool two = B > kMt2Above;
   switch (R) {
     case 64: return two ? launch_bwd<64, 2>(dhtop, whh, gates, cs, dG, S, B, st) : launch_bwd<64, 1>(dhtop, whh, gates, cs, dG, S, B, st);
     case 128: return two ? launch_bwd<128, 2>(dhtop, whh, gates, cs, dG, S, B, st) : launch_bwd<128, 1>(dhtop, whh, gates, cs, dG, S, B, st);

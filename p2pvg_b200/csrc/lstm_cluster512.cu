@@ -15,7 +15,6 @@
 //             double-buffered receive slots); the owner sums the 16 partials in a fixed order (deterministic).
 // TF32 mma.sync m16n8k8 with fp32 accumulation, MUFU activations (error <= 2^-11, below the TF32 operand rounding) exactly
 // as in lstm_cluster.cu.
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -703,15 +702,7 @@ int p2pvg_lstm_cluster512_max_clusters_impl(int which) {
 // costs about 1.5 + 2.8*MT us (measured: 4.3 / 7.1 us for MT = 1 / 2; barrier + L2 round trip, then MMA + pointwise per m16
 // tile): pick the MT with the smallest waves * step time.  B = 256: 6 clusters of 48 rows, one wave.
 static int fwd_slab_tiles(int B) {
-  static int maxc = 0, forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("P2PVG_LSTM512_MT");
-    forced = e ? atoi(e) : 0;
-    if (forced < 0 || forced > 3) forced = 0;
-    maxc = p2pvg_lstm_cluster512_max_clusters_impl(1);
-    if (maxc <= 0) maxc = 7;
-  }
-  if (forced) return forced;
+  static const int maxc = [] { const int n = p2pvg_lstm_cluster512_max_clusters_impl(1); return n > 0 ? n : 7; }();
   int best = 1;
   float best_cost = 0.f;
   for (int mt = 1; mt <= 3; mt++) {
@@ -734,18 +725,9 @@ int p2pvg_lstm_cluster512_fwd_impl(const float* pre, const float* whh, const flo
 
 // Rows per slab of the backward scan, same wave model as the forward one.  Measured per timestep: 16-row slabs (weight half in
 // shared memory) 5.7 us, 32 / 48-row slabs (weight half in tensor memory) 8.0 / 11.1 us, i.e. about 3.0 + 2.7 us per m16 tile;
-// B = 256: one wave of 6 clusters (11.2 us) instead of three waves of 16-row slabs (15.9 us).  Env override
-// P2PVG_LSTM512_BWD_MT = 1 | 2 | 3.
+// B = 256: one wave of 6 clusters (11.2 us) instead of three waves of 16-row slabs (15.9 us).
 static int bwd_slab_tiles(int B) {
-  static int maxc = 0, forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("P2PVG_LSTM512_BWD_MT");
-    forced = e ? atoi(e) : 0;
-    if (forced < 0 || forced > 3) forced = 0;
-    maxc = p2pvg_lstm_cluster512_max_clusters_impl(2);
-    if (maxc <= 0) maxc = 7;
-  }
-  if (forced) return forced;
+  static const int maxc = [] { const int n = p2pvg_lstm_cluster512_max_clusters_impl(2); return n > 0 ? n : 7; }();
   int best = 1;
   float best_cost = 0.f;
   for (int mt = 1; mt <= 3; mt++) {

@@ -27,6 +27,10 @@ import torch
 
 ACT_NONE, ACT_LRELU, ACT_TANH = 0, 1, 2
 BN_MOMENTUM = 0.1
+# BatchNorm statistics come out of a GEMM epilogue only where the tile's MMA time hides the extra epilogue work: reduction
+# length x tile width of the GEMM must reach this many MACs per output row (measured: low-K tiles are epilogue-bound and get
+# slower, DESIGN.md)
+BN_FUSE_MIN = 2048 * 128
 
 
 def skip_schedule(seq_len, probs, skip_prob, n_past):
@@ -173,38 +177,30 @@ class TrainEngine:
         self._graphs = {}
         self.dist = None  # (torch.distributed, group, world_size) when batch-sharded over several GPUs
         self.tc_lstm = tc_lstm
+        # one persistent launch per LSTM layer and direction instead of two launches per timestep, for the hidden sizes the scan
+        # kernels cover (R = 512: clusters of 16 CTAs, tensor-core mode only -- the exact-fp32 cooperative grid cannot keep a 4 MB
+        # W_hh resident)
+        self.fused_scan = hasattr(kernels, "lstm_scan_fwd") and self.R % 64 == 0 and (self.R <= 256 or (self.R == 512 and tc_lstm))
         # bf16 mode: 4x4/s2 (transposed) convolutions with >= 64 channels on both sides run as implicit GEMMs (4-D TMA
-        # pixel-box gathers), without im2col / col2im buffers; P2PVG_IMPLICIT=0 keeps the explicit lowering
-        import os
-        # one persistent cooperative launch per LSTM layer and direction instead of two launches per timestep
-        # direct CUDA-core kernels for the 1/3-channel ends: measured slower than im2col + tcgen05 GEMM, so opt-in only
-        self.thin = hasattr(kernels, "conv_thin_in") and os.environ.get("P2PVG_THIN", "0") == "1"
-        # (R = 512: clusters of 16 CTAs, tensor-core mode only -- the exact-fp32 cooperative grid cannot keep a 4 MB W_hh resident)
-        r512 = self.R == 512 and tc_lstm and os.environ.get("P2PVG_LSTM_CLUSTER", "1") != "0"
-        self.fused_scan = hasattr(kernels, "lstm_scan_fwd") and self.R % 64 == 0 and (self.R <= 256 or r512) and os.environ.get("P2PVG_FUSED_SCAN", "1") != "0"
+        # pixel-box gathers), without im2col / col2im buffers.  P2PVG_IMPLICIT=0 keeps the explicit lowering, the independent
+        # second lowering that the bf16 tests compare against.
         self.implicit = (act_dtype == torch.bfloat16) and hasattr(kernels, "conv_gemm") and os.environ.get("P2PVG_IMPLICIT", "1") != "0"
         # 1/3-channel ends (K = 16 nc or N = 16 nc < 64): four pixel rows are multiplied as one row against a block-diagonal
         # copy of the weight, so that no TMA box is out of bounds (measured 3x faster than the partially-OOB boxes)
-        self.bd = (act_dtype == torch.bfloat16) and hasattr(kernels, "blockdiag") and os.environ.get("P2PVG_BLOCKDIAG", "1") != "0"
-        # weight gradients and the skip-path of the backward pass are off the critical path: they are enqueued on a side
-        # stream (captured into the same CUDA graph) so that the TMA-bound wgrad GEMMs overlap the HBM-bound BatchNorm kernels
-        # and the latency-bound LSTM scans of the main stream.  Measured gain on one B200: 1.3 % (24.57 -> 24.26 ms) -- the
-        # persistent GEMMs leave little room for a co-resident kernel -- so it is opt-in: P2PVG_OVERLAP=1.
-        # BatchNorm forward statistics come out of the producing implicit GEMM's epilogue (per-tile column sums) instead of a
-        # separate pass over the stored tensor; P2PVG_BN_FUSE=0 keeps the stand-alone statistics kernel (A/B comparison)
-        # 1-channel stacks: tap gather + sigmoid + MSE of the last decoder layer as one kernel (no raw-output tensor)
+        self.bd = (act_dtype == torch.bfloat16) and hasattr(kernels, "blockdiag")
         # the skip-half addend of the implicit (transposed) convolutions is stored in the activation dtype: it is read once per
-        # decode call by the main GEMM's epilogue (fp32 doubled that traffic and its L2 footprint); P2PVG_ADDEND_BF16=0 = fp32
-        self.addend_dtype = act_dtype if os.environ.get("P2PVG_ADDEND_BF16", "1") != "0" else torch.float32
-        self.fuse_last = hasattr(kernels, "convt_c1_loss") and act_dtype == torch.bfloat16 and os.environ.get("P2PVG_FUSE_LAST", "1") != "0"
-        self.fuse_stats = self.implicit and os.environ.get("P2PVG_BN_FUSE", "1") != "0"
-        # ... but only where the tile's MMA time hides the extra epilogue work: reduction length x tile width of the GEMM must
-        # reach this many MACs per output row (measured: low-K tiles are epilogue-bound and get slower, DESIGN.md)
-        self.fuse_stats_min = int(os.environ.get("P2PVG_BN_FUSE_MIN", str(2048 * 128)))
-        self.overlap = getattr(kernels, "name", "") == "cuda" and os.environ.get("P2PVG_OVERLAP", "0") == "1"
-        # independent chains of small kernels (the three LSTMs, backward #2) run on side streams inside the captured graph
-        self.concurrent = getattr(kernels, "name", "") == "cuda" and act_dtype == torch.bfloat16 and os.environ.get("P2PVG_CONCURRENT", "1") != "0" \
-            and os.environ.get("P2PVG_LSTM_CLUSTER", "1") != "0"   # (the cooperative-grid scans must not share the GPU with a second grid-barrier kernel)
+        # decode call by the main GEMM's epilogue (fp32 doubled that traffic and its L2 footprint)
+        self.addend_dtype = act_dtype
+        # 1- and 3-channel bf16 stacks: tap gather + sigmoid + MSE of the last decoder layer as one kernel (no raw-output tensor)
+        self.fuse_last = hasattr(kernels, "convt_c1_loss") and act_dtype == torch.bfloat16
+        # BatchNorm forward statistics come out of the producing implicit GEMM's epilogue (per-tile column sums) instead of a
+        # separate pass over the stored tensor, where the tile shape allows it and it pays (stat_buf)
+        self.fuse_stats = self.implicit
+        # independent chains of small kernels (the prior LSTM, the LSTM weight gradients, backward #2) run on side streams
+        # inside the captured graph.  bf16 mode only: the exact-fp32 mode scans on cooperative grids, which must not share the
+        # GPU with a second grid-barrier kernel (bf16 with a hidden size the cluster scans do not cover, e.g. 192, also scans
+        # on cooperative grids and still runs the prior and posterior scans side by side).
+        self.concurrent = getattr(kernels, "name", "") == "cuda" and act_dtype == torch.bfloat16
         self.streams, self._dirty, self._serial = {}, set(), False
         # early read-back of the four scalars (P2PModel.forward): zero-copy store into page-locked host memory right after the
         # loss finalisation, polled by the host while the rest of the step is still running
@@ -221,18 +217,15 @@ class TrainEngine:
 
     # ------------------------------------------------------------------ side streams ("lanes")
     # lane 0 = the caller's stream.  lane 1: the prior LSTM while the posterior runs on lane 0 (independent recurrences until
-    # z); lane 2: weight-gradient work (never on the critical path); lane 3: backward #2 (CPC chain + prior BPTT, independent
+    # z); lane 2: LSTM weight gradients (never on the critical path); lane 3: backward #2 (CPC chain + prior BPTT, independent
     # of the encoder backward).  Every lane has its own workspaces (K.lane).  All of it is captured into the one CUDA graph.
     LANE_PRIOR, LANE_WGRAD, LANE_BWD2 = 1, 2, 3
 
-    def fork(self, lane=2, heavy=False):
+    def fork(self, lane=2):
         """Context manager: kernels enqueued inside run on side stream `lane`, after everything enqueued on the current
-        stream so far.  heavy=True marks persistent all-SM GEMMs, which gain little from a co-resident kernel: those forks
-        are only taken with P2PVG_OVERLAP=1.  Forks are only taken from lane 0 (no nesting) and never while phases are
-        being timed."""
+        stream so far.  Forks are only taken from lane 0 (no nesting) and never while phases are being timed."""
         import contextlib
-        on = self.overlap if heavy else self.concurrent
-        if not on or self.phase_events is not None or self._serial or self.K.lane != 0:
+        if not self.concurrent or self.phase_events is not None or self._serial or self.K.lane != 0:
             return contextlib.nullcontext()
         st = self.streams.get(lane)
         if st is None:
@@ -649,14 +642,11 @@ class TrainEngine:
             cn, bn = self.enc_names(l)
             imp = self.implicit and cin % 64 == 0 and cout % 64 == 0
             col = None
-            thin = self.thin and cin <= 4
             sp = None
             if imp:
                 sp = self.stat_buf(f"enc{l}", M, 1, cout, B * Ho * Ho, kred=16 * cin)
                 K.conv_gemm(0, a, self._packed[f"enc{l}"], raw, N, Ho, Ho, cin, cout, bias=P[cn + ".bias"],
                             stat_partial=sp["buf"] if sp else None)
-            elif thin:  # 1/3-channel input: direct HBM-bound kernel on the fp32 master weights
-                K.conv_thin_in(a, P[cn + ".weight"], P[cn + ".bias"], raw, N, H, H, cin, cout)
             else:
                 col = self.buf(f"enc_col{l}", M * 16 * cin)
                 K.im2col(a, col, N, H, H, cin)
@@ -665,7 +655,7 @@ class TrainEngine:
                 else:
                     K.gemm(col, self._packed[f"enc{l}"], raw, M, cout, 16 * cin, bias=P[cn + ".bias"])
             st = self.bn_forward("enc", l, raw, y, T, B * Ho * Ho, cout, P[bn + ".weight"], P[bn + ".bias"], ACT_LRELU, tiles=sp)
-            self.enc.append(dict(col=col, raw=raw, y=y, st=st, cin=cin, cout=cout, Hin=H, Hout=Ho, M=M, imp=imp, inp=a, thin=thin))
+            self.enc.append(dict(col=col, raw=raw, y=y, st=st, cin=cin, cout=cout, Hin=H, Hout=Ho, M=M, imp=imp, inp=a))
             a, H = y, Ho
         # final 4x4 valid conv == GEMM over the flattened 4x4xC map
         ctop = self.chans[-1]
@@ -695,7 +685,7 @@ class TrainEngine:
         (a 128-row tile must not straddle two BatchNorm groups) or does not pay (kred = reduction length of one tile: short
         reductions leave the epilogue no MMA time to hide behind).  rows: GEMM rows (per phase)."""
         bn_tile = 256 if C % 256 == 0 else 128 if C > 64 else 64
-        if not self.fuse_stats or rows_per_group % 128 != 0 or rows % 128 != 0 or kred * bn_tile < self.fuse_stats_min:
+        if not self.fuse_stats or rows_per_group % 128 != 0 or rows % 128 != 0 or kred * bn_tile < BN_FUSE_MIN:
             return None
         buf = self.fbuf(f"bnpart_{tag}", (rows // 128) * phases * C * 2)
         return dict(buf=buf, parts_per_group=(rows_per_group // 128) * phases, ldp=C, fold=1)
@@ -852,11 +842,6 @@ class TrainEngine:
                 sp = self.stat_buf(f"dec{k}", Md, 4, cout, B * Hi * Hi, kred=4 * cd) if k < n - 1 else None
                 K.conv_gemm(2, d, wD, raw, N, Hi, Hi, cd, cout, addend=addS, grp_src=self.ix["skip_src"], imgs_per_group=B,
                             stat_partial=sp["buf"] if sp else None)
-            elif self.thin and cout <= 3 and cd % 8 == 0:
-                w32 = P[cn + ".weight"]  # [2*cd, nc, 4, 4] fp32 master: rows [0,cd) act on d, rows [cd,2cd) on the skip
-                addS = self.fbuf(f"dec_addS{k}", nskip * B * 4 * Hi * Hi * cout)
-                K.convT_thin_out(skip, w32[cd:], P[cn + ".bias"], addS, nskip * B, Hi, Hi, cd, cout)
-                K.convT_thin_out(d, w32[:cd], None, raw, N, Hi, Hi, cd, cout, addend=addS, grp_src=self.ix["skip_src"], imgs_per_group=B)
             else:
                 colD = self.buf("dec_colD", Md * 16 * cout)
                 colS = self.buf("dec_colS", Ms * 16 * cout)
@@ -871,8 +856,7 @@ class TrainEngine:
                     rec_fused = (colD, colS, Hi, P[cn + ".bias"])
                 else:
                     K.col2im(colD, raw, N, Hi, Hi, cout, bias=P[cn + ".bias"], col2=colS, grp_src=self.ix["skip_src"], imgs_per_group=B)
-            rec = dict(inp=d, skip=skip, raw=raw, cd=cd, cout=cout, Hi=Hi, Md=Md, Ms=Ms, imp=imp, fused_loss=rec_fused,
-                       thin=(not imp) and self.thin and cout <= 3 and cd % 8 == 0)
+            rec = dict(inp=d, skip=skip, raw=raw, cd=cd, cout=cout, Hi=Hi, Md=Md, Ms=Ms, imp=imp, fused_loss=rec_fused)
             if k < n - 1:
                 dn = self.buf(f"dec_d{k}", Mo * cout)
                 rec["st"] = self.bn_forward("dec", k, raw, dn, G, B * 4 * Hi * Hi, cout, P[bn + ".weight"], P[bn + ".bias"], ACT_LRELU, tiles=sp)
@@ -941,39 +925,20 @@ class TrainEngine:
                 gw = self.fbuf(f"gwp_dec{k}", 2 * cd * 16 * cout)
             if rec["imp"]:
                 # data gradient = stride-2 conv of dy; weight gradients gather dy by filter tap; the skip half works
-                # on dy summed over the calls that share a skip frame (conv is linear) -- no col buffers at all.
-                # Only the data gradient is on the critical path: everything else goes to the side stream.
-                with self.fork(self.LANE_WGRAD, heavy=True):
-                    if want_wgrad:
-                        K.conv_gemm(1, x_in, dy, gw[:cd * 16 * cout], N, Hi, Hi, 0, cout, Cm=cd)
-                    if want_skip:
-                        dyS = self.buf(f"scratch_dyS{k}", nskip * B * Ho * Ho * cout)
-                        K.group_sum(dy, dyS, self.ix["skip_src"][g0:g1], Gn, nskip, B * Ho * Ho * cout)
-                        dsk = self.buf(f"dskip{k}", Ms * cd)
-                        K.conv_gemm(0, dyS, wS, dsk, nskip * B, Hi, Hi, cout, cd)
-                        rec["dskip"] = dsk
-                        if want_wgrad:
-                            K.conv_gemm(1, rec["skip"], dyS, gw[cd * 16 * cout:], nskip * B, Hi, Hi, 0, cout, Cm=cd)
-                    if want_wgrad:
-                        K.transpose_batched(gw, A.g[cn + ".weight"], 2 * cd, 16, cout)   # [2cd][tap][co] -> [2cd][co][tap]
-                K.conv_gemm(0, dy, wD, dd, N, Hi, Hi, cout, cd)
-            elif rec["thin"]:
-                w32 = A.p[cn + ".weight"]
-                K.conv_thin_in(dy, w32[:cd], None, dd, N, Ho, Ho, cout, cd)   # data gradient: the ConvT weight is a conv weight [cd][nc][4][4]
+                # on dy summed over the calls that share a skip frame (conv is linear) -- no col buffers at all
                 if want_wgrad:
-                    dcol = self.buf("scratch_dcol", Md * 16 * cout)
-                    K.im2col(dy, dcol, N, Ho, Ho, cout)
-                    K.gemm(x_in, dcol, gw[:cd * 16 * cout], cd, 16 * cout, Md, a_mn=True, b_mn=True, lda=cd, ldb=16 * cout)
+                    K.conv_gemm(1, x_in, dy, gw[:cd * 16 * cout], N, Hi, Hi, 0, cout, Cm=cd)
                 if want_skip:
-                    dyS = self.buf("scratch_dyS", nskip * B * Ho * Ho * cout)
+                    dyS = self.buf(f"scratch_dyS{k}", nskip * B * Ho * Ho * cout)
                     K.group_sum(dy, dyS, self.ix["skip_src"][g0:g1], Gn, nskip, B * Ho * Ho * cout)
                     dsk = self.buf(f"dskip{k}", Ms * cd)
-                    K.conv_thin_in(dyS, w32[cd:], None, dsk, nskip * B, Ho, Ho, cout, cd)
+                    K.conv_gemm(0, dyS, wS, dsk, nskip * B, Hi, Hi, cout, cd)
                     rec["dskip"] = dsk
                     if want_wgrad:
-                        dcolS = self.buf("scratch_dcolS", Ms * 16 * cout)
-                        K.im2col(dyS, dcolS, nskip * B, Ho, Ho, cout)
-                        K.gemm(rec["skip"], dcolS, gw[cd * 16 * cout:], cd, 16 * cout, Ms, a_mn=True, b_mn=True, lda=cd, ldb=16 * cout)
+                        K.conv_gemm(1, rec["skip"], dyS, gw[cd * 16 * cout:], nskip * B, Hi, Hi, 0, cout, Cm=cd)
+                if want_wgrad:
+                    K.transpose_batched(gw, A.g[cn + ".weight"], 2 * cd, 16, cout)   # [2cd][tap][co] -> [2cd][co][tap]
+                K.conv_gemm(0, dy, wD, dd, N, Hi, Hi, cout, cd)
             else:
                 dcol = self.buf("scratch_dcol", Md * 16 * cout)
                 K.im2col(dy, dcol, N, Ho, Ho, cout)
@@ -995,8 +960,8 @@ class TrainEngine:
                     rec["dskip"] = dsk
                     if want_wgrad:
                         K.gemm(rec["skip"], dcolS, gw[cd * 16 * cout:], cd, 16 * cout, Ms, a_mn=True, b_mn=True, lda=cd, ldb=16 * cout)
-            if want_wgrad and not rec["imp"]:
-                K.transpose_batched(gw, A.g[cn + ".weight"], 2 * cd, 16, cout)   # [2cd][tap][co] -> [2cd][co][tap]
+                if want_wgrad:
+                    K.transpose_batched(gw, A.g[cn + ".weight"], 2 * cd, 16, cout)   # [2cd][tap][co] -> [2cd][co][tap]
             dy = dd
         # upc1: BatchNorm + LeakyReLU, then the g -> 4x4xCtop GEMM
         ctop = self.chans[-1]
@@ -1161,7 +1126,8 @@ class TrainEngine:
         A = self.arena["encoder"]
         N = T * B
         nskip = plan.nskip
-        self.join(self.LANE_WGRAD)   # the skip gradients of the decoder come from the side stream
+        # lane 0 waits for the LSTM weight gradients (a no-op in single-GPU mode A, whose Adam step has joined every lane)
+        self.join(self.LANE_WGRAD)
         if self.adt == torch.float32:
             dy = self.dH
         else:
@@ -1194,17 +1160,10 @@ class TrainEngine:
             A.g[cn + ".bias"].zero_()
             gw = self.fbuf(f"gwp_enc{l}", cout * 16 * cin)
             if rec["imp"]:
-                with self.fork(self.LANE_WGRAD, heavy=True):   # off the critical path
-                    K.conv_gemm(1, gy, rec["inp"], gw, N, Ho, Ho, 0, cin, Cm=cout)
-                    K.transpose_batched(gw, A.g[cn + ".weight"], cout, 16, cin)   # [co][tap][ci] -> [co][ci][tap]
+                K.conv_gemm(1, gy, rec["inp"], gw, N, Ho, Ho, 0, cin, Cm=cout)
             else:
-                col = rec["col"]
-                if col is None:  # thin first layer: the im2col matrix is only needed here
-                    col = self.buf(f"enc_col{l}", M * 16 * cin)
-                    K.im2col(rec["inp"], col, N, rec["Hin"], rec["Hin"], cin)
-                K.gemm(gy, col, gw, cout, 16 * cin, M, a_mn=True, b_mn=True, lda=cout, ldb=16 * cin)
-            if not rec["imp"]:
-                K.transpose_batched(gw, A.g[cn + ".weight"], cout, 16, cin)   # [co][tap][ci] -> [co][ci][tap]
+                K.gemm(gy, rec["col"], gw, cout, 16 * cin, M, a_mn=True, b_mn=True, lda=cout, ldb=16 * cin)
+            K.transpose_batched(gw, A.g[cn + ".weight"], cout, 16, cin)   # [co][tap][ci] -> [co][ci][tap]
             if l > 0:
                 gprev = self.buf(f"enc_gy{l - 1}", N * rec["Hin"] * rec["Hin"] * cin)
                 if rec["imp"]:

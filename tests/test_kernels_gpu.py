@@ -287,6 +287,31 @@ def test_batchnorm_matches_torch(KS):
         close(y[g].reshape(B, H, H, C).permute(0, 3, 1, 2), ref, rtol=1e-4, atol=1e-5)
 
 
+@pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
+def test_bn_bwd_without_activation_tensor(KS, dtype):
+    K, _ = KS
+    torch.manual_seed(2)
+    G, R, C = 3, 200, 64
+    x = (torch.randn(G, R, C, device="cuda") * 2 + 0.3).to(dtype)
+    gamma, beta = torch.randn(C, device="cuda") * 0.1 + 1, torch.randn(C, device="cuda") * 0.1
+    st = [torch.zeros(G * C, device="cuda") for _ in range(5)]
+    K.bn_fwd_stats(x, G, R, C, gamma, beta, *st)
+    y = torch.empty_like(x)
+    K.bn_act(x, y, st[3], st[4], G, R, C, 1)
+    dy = torch.randn(G, R, C, device="cuda").to(dtype)
+    outs = []
+    for use_y in (True, False):
+        dx = torch.empty_like(x)
+        s0, s1 = torch.zeros(G * C, device="cuda"), torch.zeros(G * C, device="cuda")
+        if use_y:
+            K.bn_bwd(dy, x, y, st[0], st[1], gamma, G, R, C, 1, dx, s0, s1)
+        else:
+            K.bn_bwd(dy, x, None, st[0], st[1], gamma, G, R, C, 1, dx, s0, s1, scale=st[3], shift=st[4])
+        outs.append((dx, s0, s1))
+    for a, b in zip(*outs):
+        assert torch.equal(a, b) or (a.float() - b.float()).abs().max().item() <= 1e-6
+
+
 def test_lstm_pointwise_and_reparam(KS):
     Kc, Ke = KS
     B, R = 7, 256

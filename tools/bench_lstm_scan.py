@@ -1,5 +1,6 @@
 #!/usr/bin/env python
-"""CUDA-event timing of the persistent LSTM scan kernels (P2PVG_LSTM_CLUSTER=0|1 selects the implementation)."""
+"""CUDA-event timing of the persistent LSTM scan kernels: tf32 = 1 runs the thread-block-cluster scans for R in {64,128,256,512},
+tf32 = 0 (or any other R) the cooperative-grid scans."""
 import os
 import sys
 
